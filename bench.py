@@ -2,7 +2,7 @@
 """bench.py — env-steps/s of the batched HighwayEnv hot path on B200, every BASELINE.json config in one line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--envs-per-gpu E] [--configs cfg2,cfg3] [--gather-obs] [--no-cpu-baseline]
+                    [--envs-per-gpu E] [--configs cfg2,cfg3] [--gather-obs] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Headline (top-level keys of the JSON line) = BASELINE.json configs[1]: highway-fast-v0, vehicles_count=50
 (V = 51), 3 lanes, 5 substeps per step, Kinematics observation, DiscreteMetaAction, 4096 envs per GPU
@@ -26,6 +26,10 @@ with --gather-obs, the cost of the optional NCCL all-gather of the whole-batch o
                "measured elsewhere", the per-core rate of the UNMODIFIED Python reference from
                profiles/r2_python_reference.json (tools/time_reference.py, build container).
 
+--dump-outputs DIR: after the timed steps, what the last timed env.step of every config returned to its caller
+(observation, reward, terminated, truncated and the info arrays) as DIR/<config>_<name>.npy in float32 / float64, rank 0's
+envs only; the inputs (reset seeds, action streams) are fixed, so two builds can be compared output for output.
+
 --impl reference: the CPU arm of the headline config alone (the Python reference cannot travel to the GPU
 box: /root/reference is absent there and gymnasium is not installed; the C port is its line-cited restatement).
 """
@@ -47,6 +51,7 @@ METRIC = "env-steps/sec (batched), highway-fast-v0 50 veh"
 UNIT = "env-steps/s"
 HEADLINE = "cfg2"
 STRONG_TOTAL_ENVS = 32768
+DUMP_LIMIT_BYTES = 64 << 20  # --dump-outputs: above this, a fixed seeded sample of the envs is written
 
 # SURVEY.md §8(d): algorithmic bytes per env-step = 2*V*B_state + B_action + B_obs + 6
 CONFIGS = {
@@ -462,8 +467,41 @@ def _make_actions(kind, shape_n, count, gen, dev, torch):
     return torch.randint(0, hi, (count, shape_n), generator=gen, device=dev, dtype=torch.int32)
 
 
-def measure_config(key, E, K, W, rank, world, dev, ctx, do_e2e=True, gather=False):
-    """Device-timed and end-to-end throughput of one config on this rank; returns local timings."""
+def _host_arrays(x, name: str, out: dict) -> None:
+    """The tensors of an env.step return value (nested in tuples / dicts) as float32 / float64 numpy arrays."""
+    import numpy as np
+    import torch
+
+    if isinstance(x, (dict, tuple, list)):
+        for k, v in (x.items() if isinstance(x, dict) else enumerate(x)):
+            _host_arrays(v, f"{name}_{k}" if name else str(k), out)
+    elif isinstance(x, torch.Tensor):
+        a = x.detach().cpu().numpy()
+        out[name] = a if a.dtype.kind == "f" and a.itemsize >= 4 else a.astype(np.float32 if a.dtype.kind == "b" else np.float64)
+
+
+def dump_outputs(outputs: dict, path: str) -> None:
+    """outputs: config -> {name: array [envs, ...]}.  Writes <path>/<config>_<name>.npy; if the whole exceeds
+    DUMP_LIMIT_BYTES, every config keeps the same fraction of its envs, chosen by a fixed seed (written as
+    <config>_env_index.npy)."""
+    import numpy as np
+
+    total = sum(a.nbytes for arrays in outputs.values() for a in arrays.values())
+    frac = min(1.0, DUMP_LIMIT_BYTES / total) if total else 1.0
+    os.makedirs(path, exist_ok=True)
+    for key, arrays in outputs.items():
+        n = len(next(iter(arrays.values())))
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(0).permutation(n)[:max(1, int(n * frac * 0.99))])
+            arrays = {name: a[idx] for name, a in arrays.items()}
+            arrays["env_index"] = idx.astype(np.float64)
+        for name, a in arrays.items():
+            np.save(os.path.join(path, f"{key}_{name}.npy"), a)
+
+
+def measure_config(key, E, K, W, rank, world, dev, ctx, do_e2e=True, gather=False, dump=False):
+    """Device-timed and end-to-end throughput of one config on this rank; returns local timings (and, with
+    `dump`, the host copies of what the last timed step returned, under "outputs")."""
     import torch
     import torch.distributed as dist
 
@@ -504,17 +542,23 @@ def measure_config(key, E, K, W, rank, world, dev, ctx, do_e2e=True, gather=Fals
     for k in range(K):
         flush.fill_(k & 0xFF)  # > L2: the state is read from HBM in every timed step
         ev[k][0].record(stream)
-        env.step(actions[W + k])
+        last = env.step(actions[W + k])
         ev[k][1].record(stream)
     barrier()
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if sampler else None
+    outputs = {}
+    if dump:  # before the e2e and road-only passes below reuse the env's output buffers
+        _host_arrays(dict(zip(("obs", "reward", "terminated", "truncated", "info"), last)), "", outputs)
+    del last
     launches = int(lib.hwy_launch_count() - launches0)
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     kev, env._kernel_events = env._kernel_events, None
     kern_ms = sum(a.elapsed_time(b) for a, b in kev) / max(1, len(kev)) if kev else total_ms / K
     res = {"total_ms": total_ms, "kern_ms": kern_ms, "launches": launches, "wall_s": t_wall, "clocks": clocks,
            "obs_bytes": int(env._obs[0].numel() * 4), "act_bytes": int(actions[0].numel() * actions.element_size() // E)}
+    if dump:
+        res["outputs"] = outputs
 
     if gather and world > 1:
         from highwayenv_b200.parallel import all_gather_batch
@@ -642,11 +686,14 @@ def run_gpu_arm(args) -> None:
             dist.all_reduce(t)
         return int(t.item())
 
-    entries, head, head_raw = [], None, None
+    entries, head, head_raw, outputs = [], None, None, {}
     for key in keys:
         E = envs_for(key)
-        Kc = K if key == HEADLINE else max(20, min(K, args.other_steps))
-        r = measure_config(key, E, Kc, W, rank, world, dev, ctx, gather=args.gather_obs and key == HEADLINE)
+        Kc = K if key == HEADLINE or not args.other_steps else args.other_steps
+        r = measure_config(key, E, Kc, W, rank, world, dev, ctx, gather=args.gather_obs and key == HEADLINE,
+                           dump=bool(args.dump_outputs) and rank == 0)
+        if "outputs" in r:
+            outputs[key] = r.pop("outputs")
         total_ms, e2e_s, e2e_eager, kern_ms = reduce_max([r["total_ms"], r["e2e_s"], r["e2e_eager_s"], r["kern_ms"]])
         launches = reduce_sum(r["launches"])
         n_total = E * world
@@ -705,6 +752,8 @@ def run_gpu_arm(args) -> None:
                   "step_ms_without": head["ms_per_step"]}
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(outputs, args.dump_outputs)
         if not args.no_cpu_baseline:
             for entry in entries:
                 cb = cpu_arm(entry["id"], args.cpu_seconds, 3)
@@ -743,10 +792,10 @@ def run_gpu_arm(args) -> None:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100, help="timed steps of every config")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--envs-per-gpu", type=int, default=0, help="override for the headline config")
-    ap.add_argument("--other-steps", type=int, default=50, help="timed steps of the non-headline configs")
+    ap.add_argument("--other-steps", type=int, default=0, help="timed steps of the non-headline configs (default: --steps)")
     ap.add_argument("--configs", default="", help="comma list (cfg1..cfg5); default all")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -755,7 +804,11 @@ def main() -> None:
     ap.add_argument("--cpu-seconds", type=float, default=3.0)
     ap.add_argument("--cpu-repeats", type=int, default=3)
     ap.add_argument("--cpu-arm", default="", help="internal: run the CPU arm of one config and print its JSON")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step of every config returned as DIR/<config>_<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.other_steps < 0:
+        ap.error("--steps must be >= 1 and --other-steps >= 0")
     if args.cpu_arm:
         print(json.dumps(cpu_arm_inprocess(args.cpu_arm, args.cpu_seconds, args.cpu_repeats)), flush=True)
         return

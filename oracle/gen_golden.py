@@ -1,6 +1,8 @@
 """Generate golden fixtures from the UNMODIFIED Python reference (build container only).
 
-    python oracle/gen_golden.py            # writes tests/golden/*.npz
+    python oracle/gen_golden.py              # writes tests/golden/*.npz
+    python oracle/gen_golden.py obs_plugins  # tests/golden/obs_plugins_*.npz
+    python oracle/gen_golden.py live         # tests/golden/live_*: what the tests/test_*_live.py tests compare against
 
 Each fixture is a seeded rollout of the reference env (ref_harness.rollout): the full
 per-vehicle state after reset and after every env.step, plus obs / reward / terminated /
@@ -251,6 +253,240 @@ def gen_obs_plugins(only) -> None:
         print(f"{name}: {len(states)} states x {len(obs_cfgs)} observation types -> {path} ({os.path.getsize(path)/1e3:.0f} kB)")
 
 
+# ------------------------------------------------------------------ fixtures of tests/test_*_live.py
+# What those tests compare the oracles against, recorded from the reference on their own seeds (seeds in no fixture
+# above) so that they run without it: tests/golden/live_<case>.npz and tests/golden/live_network_configs.json.
+LIVE_HIGHWAY = {  # tests/test_oracle_live.py: teacher-forced, one env
+    "highway-fast-v0": ({"vehicles_count": 50}, 12, 4242),
+    "highway-v0": ({"vehicles_count": 30, "lanes_count": 5, "action": {"type": "ContinuousAction"}}, 6, 77),
+}
+LIVE_NET = {  # tests/test_net_oracle_live.py: teacher-forced, one env per seed
+    "roundabout-v0": ({"observation": {"type": "TimeToCollision", "horizon": 10}}, 11, (31, 32)),
+    "roundabout-v1": (None, 11, (33,)),
+    "merge-v0": (None, 14, (34, 35)),
+    "merge-v1": (None, 14, (36,)),
+    "two-way-v0": (None, 10, (37, 38)),
+    "u-turn-v0": (None, 10, (39, 40)),
+    "u-turn-v1": (None, 10, (41,)),
+}
+LIVE_INTERSECTION = {  # tests/test_intersection_oracle_live.py: free-running, one env per seed
+    ("intersection-v0", "default"): (5000, 6), ("intersection-v0", "OccupancyGrid"): (5100, 6),
+    ("intersection-v2", "default"): (5200, 4), ("intersection-multi-agent-v0", "default"): (5300, 4),
+}
+LIVE_NETWORK_BUILDERS = {  # tests/test_network_config_live.py: RoadNetwork.to_config / from_config
+    "roundabout-v0": ("highwayenv_b200.envs.roundabout_env", "make_roundabout_network"),
+    "intersection-v0": ("highwayenv_b200.envs.intersection_env", "make_intersection_network"),
+    "merge-v0": ("highwayenv_b200.envs.merge_env", "make_merge_network"),
+    "two-way-v0": ("highwayenv_b200.envs.two_way_env", "make_two_way_network"),
+    "u-turn-v0": ("highwayenv_b200.envs.u_turn_env", "make_u_turn_network"),
+}
+
+
+def live_name(env_id: str, obs: str = "") -> str:
+    return "live_" + env_id.replace("-", "_") + ("_" + obs if obs and obs != "default" else "")
+
+
+def _save(name: str, out: dict) -> None:
+    path = os.path.join(OUT, name + ".npz")
+    np.savez_compressed(path, **out)
+    print(f"{name} -> {path} ({os.path.getsize(path)/1e3:.0f} kB)")
+
+
+def _rng_words(env) -> np.ndarray:
+    m64, st = (1 << 64) - 1, env.np_random.bit_generator.state
+    return np.array([st["state"]["state"] >> 64, st["state"]["state"] & m64, st["state"]["inc"] >> 64,
+                     st["state"]["inc"] & m64, (int(st["has_uint32"]) << 32) | int(st["uinteger"])], dtype=np.uint64)
+
+
+def _stack_states(states: list, prefix: str = "") -> dict:
+    """dump_state dicts -> {prefix + key: array stacked over steps}."""
+    return {prefix + k: np.stack([s[k] for s in states]) for k in states[0]}
+
+
+def _shared(out: dict, seed: int, env, cfg: dict) -> None:
+    """The road network and config, stored once per file: the same for every seed of a case."""
+    import json
+
+    net = rh.dump_network(env)
+    net["config_json"] = np.array(json.dumps(cfg))
+    if "config_json" not in out:
+        out.update(net)
+    for k, v in net.items():
+        assert np.array_equal(out[k], v), (seed, k)
+
+
+def gen_live_highway(env_id: str) -> None:
+    import json
+
+    over, T, seed = LIVE_HIGHWAY[env_id]
+    rng = np.random.default_rng(seed)  # the test's action draws, in its order
+    cont = (over or {}).get("action", {}).get("type") == "ContinuousAction"
+    actions = [rng.uniform(-1, 1, size=2).astype(np.float32) if cont else int(rng.integers(5)) for _ in range(T)]
+    out = rh.rollout(env_id, over, seed, actions)
+    out["config_json"] = np.array(json.dumps(dict(rh.make_reference_env(env_id, over).config)))
+    _save(live_name(env_id), out)
+
+
+def gen_live_available_actions() -> None:
+    """DiscreteMetaAction.get_available_actions (action.py:262-299) on 200 scripted ego placements."""
+    env = rh.make_reference_env("highway-fast-v0", {"lanes_count": 3})
+    env.reset(seed=0)
+    rng = np.random.default_rng(0)
+    rows, masks = [], []
+    for _ in range(200):
+        v = env.vehicle
+        lane, si = int(rng.integers(3)), int(rng.integers(3))
+        x = float(rng.choice([-3.0, 0.0, 50.0, 9999.0, 10004.99, 10005.0, 10010.0]))
+        y = 4.0 * lane + float(rng.uniform(-2, 2))
+        v.position, v.lane_index, v.speed_index = np.array([x, y]), ("0", "1", lane), si
+        v.lane = env.road.network.get_lane(v.lane_index)
+        m = np.zeros(5, dtype=np.bool_)
+        m[sorted(set(env.action_type.get_available_actions()))] = True
+        rows.append((x, y, lane, si))
+        masks.append(m)
+    r = np.array(rows, dtype=np.float64)
+    _save("live_available_actions", {"x": r[:, 0], "y": r[:, 1], "lane": r[:, 2].astype(np.int64),
+                                     "speed_index": r[:, 3].astype(np.int64), "mask": np.stack(masks)})
+
+
+def gen_live_net(env_id: str) -> None:
+    """Per seed, keys prefixed s<seed>_: the state after reset and every step (the vehicle count may differ by seed)."""
+    over, T, seeds = LIVE_NET[env_id]
+    out = {"seeds": np.array(seeds, dtype=np.int64)}
+    for seed in seeds:
+        env = rh.make_reference_env(env_id, over)
+        obs_ref, _ = env.reset(seed=seed)
+        cfg = dict(env.config)
+        cfg["_env_id"] = env_id
+        if env_id.startswith("merge"):
+            lanes = [li for li, _ in rh.lane_list(env)]
+            cfg["_merge_lane"] = lanes.index(("b", "c", 2))
+            cfg["_default_side_lanes"] = len(env.road.network.all_side_lanes(env.vehicle.lane_index))
+        _shared(out, seed, env, cfg)
+        p = f"s{seed}_"
+        states, obs, rew, term, trunc, acts = [rh.dump_state(env)], [np.asarray(obs_ref)], [], [], [], []
+        rng = np.random.default_rng(seed)  # the test's action draws
+        for _ in range(T):
+            a = int(rng.integers(5))
+            o, r, te, tr, _ = env.step(a)
+            states.append(rh.dump_state(env))
+            obs.append(np.asarray(o))
+            rew.append(float(r))
+            term.append(bool(te))
+            trunc.append(bool(tr))
+            acts.append(a)
+        out.update(_stack_states(states, p))
+        out[p + "obs"], out[p + "reward"] = np.stack(obs), np.array(rew, dtype=np.float64)
+        out[p + "terminated"], out[p + "truncated"] = np.array(term), np.array(trunc)
+        out[p + "actions"] = np.array(acts, dtype=np.int64)
+    _save(live_name(env_id), out)
+
+
+def gen_live_intersection(env_id: str, obs_type: str) -> None:
+    """The reference's side of the free-running comparison: every step until the episode ends or a non-crashed vehicle
+    crawls below 1 m/s (tests/parity_utils.py well_conditioned; that step is kept, the test stops before comparing it).
+    The seeds' records are concatenated along the step axis; n_steps[i] is the number of steps of seed i."""
+    seed0, n = LIVE_INTERSECTION[(env_id, obs_type)]
+    over = None if obs_type == "default" else {"observation": {"type": obs_type}}
+    out, per_seed = {"seeds": np.arange(seed0, seed0 + n, dtype=np.int64)}, []
+    for seed in range(seed0, seed0 + n):
+        env = rh.make_reference_env(env_id, over)
+        obs_ref, _ = env.reset(seed=seed)
+        cfg = dict(env.config)
+        A = int(cfg.get("controlled_vehicles", 1))
+        _shared(out, seed, env, cfg)
+        states, obs, rew, term, trunc, acts, words = [rh.dump_state(env, 32)], [np.asarray(obs_ref)], [], [], [], [], []
+        rng = np.random.default_rng(seed)  # the test's action draws
+        for _ in range(int(cfg["duration"] * cfg["policy_frequency"]) + 1):
+            a = rng.integers(0, 3, size=A)
+            o, r, te, tr, _ = env.step(tuple(int(x) for x in a) if A > 1 else int(a[0]))
+            st = rh.dump_state(env, 32)
+            states.append(st)
+            obs.append(np.asarray(o, dtype=np.float64))
+            rew.append(float(r))
+            term.append(bool(te))
+            trunc.append(bool(tr))
+            acts.append(a)
+            words.append(_rng_words(env))
+            k = int(st["count"])
+            if np.any(~st["crashed"][:k].astype(bool) & (np.abs(st["speed"][:k]) < 1.0)) or te or tr:
+                break
+        d = _stack_states(states)  # T + 1 states
+        d["obs"] = np.stack(obs)
+        d["reward"], d["terminated"], d["truncated"] = np.array(rew, dtype=np.float64), np.array(term), np.array(trunc)
+        d["actions"], d["rng_words"] = np.stack(acts).astype(np.int64), np.stack(words)
+        per_seed.append(d)
+    out.update({k: np.concatenate([d[k] for d in per_seed]) for k in per_seed[0]})
+    out["n_steps"] = np.array([len(d["reward"]) for d in per_seed], dtype=np.int64)
+    _save(live_name(env_id, obs_type), out)
+
+
+def _plain(x):
+    """A to_config() dict as JSON: arrays and tuples -> lists, numpy scalars -> python."""
+    if isinstance(x, dict):
+        return {k: _plain(v) for k, v in x.items()}
+    if isinstance(x, np.ndarray):
+        return x.tolist()
+    if isinstance(x, (list, tuple)):
+        return [_plain(v) for v in x]
+    return x.item() if isinstance(x, np.generic) else x
+
+
+def gen_live_network_config(env_id: str) -> None:
+    """The reference's RoadNetwork.to_config() of the env's road, and what its RoadNetwork.from_config makes of the
+    product's to_config() (the dict it was given is stored with it)."""
+    import importlib
+    import json
+
+    from highway_env.road.road import RoadNetwork
+
+    mod, fn = LIVE_NETWORK_BUILDERS[env_id]
+    ours = getattr(importlib.import_module(mod), fn)().to_config()
+    env = rh.make_reference_env(env_id, None)
+    env.reset(seed=0)
+    rec = {"reference": _plain(env.road.network.to_config()), "given": _plain(ours),
+           "given_round_trip": _plain(RoadNetwork.from_config(ours).to_config())}
+    path = os.path.join(OUT, "live_network_configs.json")
+    allrec = {}
+    if os.path.exists(path):
+        with open(path) as f:
+            allrec = json.load(f)
+    allrec[env_id] = rec
+    with open(path, "w") as f:
+        json.dump({k: allrec[k] for k in sorted(allrec)}, f, indent=None, separators=(",", ":"))
+        f.write("\n")
+    print(f"live_network_configs[{env_id}] -> {path}")
+
+
+def gen_live(only) -> None:
+    """Every case in a fresh interpreter: IntersectionEnv._make_vehicles rewrites IDMVehicle class constants for the
+    whole process (envs/intersection_env.py:262-265)."""
+    import subprocess
+
+    cases = ([("highway", e) for e in LIVE_HIGHWAY] + [("available_actions", "")] + [("net", e) for e in LIVE_NET]
+             + [("intersection", f"{e}:{o}") for e, o in LIVE_INTERSECTION]
+             + [("network_config", e) for e in LIVE_NETWORK_BUILDERS])
+    for kind, arg in cases:
+        if only and kind not in only:
+            continue
+        subprocess.check_call([sys.executable, os.path.abspath(__file__), "live-case", kind, arg])
+
+
+def gen_live_case(kind: str, arg: str) -> None:
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    rh._ensure_imports()
+    if kind == "highway":
+        gen_live_highway(arg)
+    elif kind == "available_actions":
+        gen_live_available_actions()
+    elif kind == "net":
+        gen_live_net(arg)
+    elif kind == "intersection":
+        gen_live_intersection(*arg.split(":"))
+    else:
+        gen_live_network_config(arg)
+
+
 if __name__ == "__main__":
     if not rh.reference_available():
         raise SystemExit("reference not mounted; golden fixtures can only be generated in the build container")
@@ -258,5 +494,9 @@ if __name__ == "__main__":
     if args and args[0] == "obs_plugins":
         rh._ensure_imports()
         gen_obs_plugins(args[1:])
+    elif args and args[0] == "live":
+        gen_live(args[1:])
+    elif args and args[0] == "live-case":
+        gen_live_case(args[1], args[2] if len(args) > 2 else "")
     else:
         main()

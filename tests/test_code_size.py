@@ -13,9 +13,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.skipif(shutil.which("nvcc") is None or shutil.which("nvdisasm") is None, reason="needs nvcc + nvdisasm")
-def test_highway_substep_loop_fits_the_instruction_cache_budget():
+def test_highway_substep_loop_fits_the_instruction_cache_budget(tmp_path):
     out = subprocess.run(["bash", os.path.join(ROOT, "tools", "loop_size.sh")], cwd=ROOT, capture_output=True, text=True,
-                         timeout=600)
+                         timeout=600, env=dict(os.environ, HWY_LOOP_SIZE_DIR=str(tmp_path)))
     assert out.returncode == 0, out.stderr[-800:]
     line = [l for l in out.stdout.splitlines() if "backward spans:" in l][-1]
     total = int(line.split(" total ")[1].split(" B;")[0])

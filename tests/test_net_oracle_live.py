@@ -1,18 +1,17 @@
-"""Network oracle vs the LIVE reference on seeds that are not in the golden fixtures (only where /root/reference
-is mounted: the build container; skipped on the GPU box).  Teacher-forced, one env at a time.  intersection ids are
-left to the fixtures: IntersectionEnv._make_vehicles rewrites IDMVehicle class constants for the whole process."""
+"""Network oracle vs the reference on seeds that are not in the other golden fixtures: what the reference computed on
+them is recorded in tests/golden/live_*.npz (`python oracle/gen_golden.py live`).  Teacher-forced, one env at a time.
+intersection ids are in tests/test_intersection_oracle_live.py (free-running)."""
 import numpy as np
 import pytest
 
 import net_oracle as no
-import ref_harness as rh
-from parity_utils import compare_state
+from parity_utils import compare_state, load_golden
 
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="reference not mounted")
+NOT_STATE = ("obs", "reward", "terminated", "truncated", "actions")
 
 
-def _state(env, V):
-    st = rh.dump_state(env)
+def _state(st, V):
+    st = dict(st)
     st["target_lane"] = np.where(st["target_lane"] < 0, st["lane"], st["target_lane"])
     if "route" not in st:
         st["route"], st["route_len"] = np.zeros((V, no.NET_MAX_ROUTE), dtype=np.int32), np.zeros(V, dtype=np.int32)
@@ -36,30 +35,28 @@ def _state(env, V):
     ("u-turn-v1", None, 10, (41,)),
 ])
 def test_net_oracle_matches_live_reference(env_id, over, T, seeds):
+    g = load_golden("live_" + env_id.replace("-", "_"))
+    assert tuple(g["seeds"]) == seeds
+    cfg = g["config"]
+    assert cfg["_env_id"] == env_id and (over is None or cfg["observation"]["type"] == over["observation"]["type"])
+    graph = no.graph_from_arrays(g)
     for seed in seeds:
-        env = rh.make_reference_env(env_id, over)
-        obs_ref, _ = env.reset(seed=seed)
-        cfg = dict(env.config)
-        cfg["_env_id"] = env_id
-        if env_id.startswith("merge"):
-            lanes = [li for li, _ in rh.lane_list(env)]
-            cfg["_merge_lane"] = lanes.index(("b", "c", 2))
-            cfg["_default_side_lanes"] = len(env.road.network.all_side_lanes(env.vehicle.lane_index))
-        V = len(env.road.vehicles) + len(env.road.objects)
-        graph = no.graph_from_arrays(rh.dump_network(env))
-        oc = no.cfg_from_dict(cfg, n_vehicles=V)
-        ob = no.NetOracleBatch(graph, oc, 1)
-        ob.load_state(0, _state(env, V))
-        assert np.max(np.abs(ob.observe().reshape(np.asarray(obs_ref).shape) - obs_ref)) <= 1e-6
-        rng = np.random.default_rng(seed)
+        p = f"s{seed}_"
+        r = {k[len(p):]: v for k, v in g.items() if k.startswith(p)}
+        assert len(r["reward"]) == T
+        states = [{k: r[k][t] for k in r if k not in NOT_STATE} for t in range(T + 1)]
+        V = len(states[0]["x"])
+        ob = no.NetOracleBatch(graph, no.cfg_from_dict(cfg, n_vehicles=V), 1)
+        ob.load_state(0, _state(states[0], V))
+        assert np.max(np.abs(ob.observe().reshape(r["obs"][0].shape) - r["obs"][0])) <= 1e-6
         for t in range(T):
-            ob.load_state(0, _state(env, V))  # teacher-forced
-            a = int(rng.integers(5))
-            o, r, te, tr, _ = env.step(a)
-            oo, ro, teo, tro = ob.step([a])
+            ob.load_state(0, _state(states[t], V))  # teacher-forced
+            oo, ro, teo, tro = ob.step([int(r["actions"][t])])
             got = {k: ob.a[k][0] for k in ob.a if k not in ("speed_index", "time")}
             got["speed_index"] = ob.a["speed_index"][0]
             ctx = f"{env_id} seed {seed} t={t}"
-            assert compare_state(_state(env, V), got, ctx=ctx) < 1e-9
-            assert abs(r - ro[0]) < 1e-9 and te == bool(teo[0]) and tr == bool(tro[0]), ctx
-            assert np.max(np.abs(np.asarray(o) - oo[0].reshape(np.asarray(o).shape))) <= 1e-6, ctx
+            assert compare_state(_state(states[t + 1], V), got, ctx=ctx) < 1e-9
+            assert abs(r["reward"][t] - ro[0]) < 1e-9, ctx
+            assert bool(r["terminated"][t]) == bool(teo[0]) and bool(r["truncated"][t]) == bool(tro[0]), ctx
+            o = r["obs"][t + 1]
+            assert np.max(np.abs(o - oo[0].reshape(o.shape))) <= 1e-6, ctx

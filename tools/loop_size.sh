@@ -1,22 +1,23 @@
 #!/bin/bash
 # Static size of a kernel and the spans of its loops (backward branches), from a cubin compiled without a GPU:
 #   bash tools/loop_size.sh [source.cu] [mangled-name substring] [extra nvcc flags...]
-# defaults: hwy_highway.cu, highway_step_kernelILi64ELb1.  Writes /tmp/hwy_loop_size/kernel.dis for sass_footprint.py.
+# defaults: hwy_highway.cu, highway_step_kernelILi64ELb1.  Writes $HWY_LOOP_SIZE_DIR/kernel.dis (default
+# /tmp/hwy_loop_size) for sass_footprint.py.
 set -e
 SRC=${1:-hwy_highway.cu}; PAT=${2:-highway_step_kernelILi64ELb1}; shift 2 2>/dev/null || true
-OUT=/tmp/hwy_loop_size; mkdir -p $OUT
+export OUT=${HWY_LOOP_SIZE_DIR:-/tmp/hwy_loop_size}; mkdir -p "$OUT"
 nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -fmad=false -cubin "$@" \
-  -o $OUT/k.cubin highwayenv_b200/csrc/$SRC
-nvdisasm -g $OUT/k.cubin > $OUT/all.dis
+  -o "$OUT/k.cubin" highwayenv_b200/csrc/$SRC
+nvdisasm -g "$OUT/k.cubin" > "$OUT/all.dis"
 PAT=$PAT python - <<'P'
 import os, re
-pat=os.environ['PAT']
-L=open('/tmp/hwy_loop_size/all.dis').read().split('\n')
+pat, out = os.environ['PAT'], os.environ['OUT']
+L=open(os.path.join(out, 'all.dis')).read().split('\n')
 starts=[k for k,l in enumerate(L) if l.startswith('\t.section\t.text.')]
 for a,b in zip(starts,starts[1:]+[len(L)]):
     name=L[a].split('.text.')[1].split(',')[0]
     if pat not in name: continue
-    open('/tmp/hwy_loop_size/kernel.dis','w').write('\n'.join(L[a:b]))
+    open(os.path.join(out, 'kernel.dis'),'w').write('\n'.join(L[a:b]))
     labels={}; ins=[]
     for l in L[a:b]:
         m=re.match(r'(\.L_x_\d+):',l)
